@@ -9,6 +9,8 @@ N > 1 (torchrun, one rank per GPU): ONE clip of 200*N frames is sharded by conti
 GPU (weak scaling), exactly: +-40-frame halo exchange before each of the 10 temporal attentions (ncclSend/Recv) and a
 16-double all-reduce per GroupNorm (40 per step) inside the library; `value` counts 200-frame-clip equivalents
 (frames denoised per second / 200).  `--replicas` runs one independent 200-frame clip per GPU instead.
+`--dump-outputs DIR` writes the eps of the last timed step as DIR/eps.npy (DIR/eps_rank<r>.npy per rank when N > 1); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 Prints ONE JSON line on rank 0.
 """
 import argparse
@@ -20,13 +22,16 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                     # the tree may be read-only: no __pycache__ for the project's modules
 
 F_CLIP, H_LAT, W_LAT = 200, 64, 64
 METRIC = "denoising-steps/sec (200-frame 256^2 clip)"
+DUMP_BYTES = 64 << 20                              # --dump-outputs: at most this much over all ranks
 CTOR = dict(dim=64, cond_dim=1032, cond_aud=1024, cond_pose=6, cond_eye=2, num_frames=40, channels=275,
             out_grid_dim=2, out_conf_dim=1, dim_mults=(1, 2, 4, 8), use_hubert_audio_cond=True,
             learn_null_cond=False, use_final_activation=False, use_deconv=True, padding_mode="zeros", win_width=40)
@@ -90,6 +95,18 @@ class ClockSampler:
 
 def log(msg):
     print(f"[bench +{time.perf_counter() - T_START:7.1f}s] {msg}", file=sys.stderr, flush=True)
+
+
+def dump_output(path, name, t, budget):
+    """`t` as path/<name>.npy in float32.  Above `budget` bytes only every k-th element of the flattened tensor is written: a fixed
+    sample, the same on every run."""
+    a = t.detach().float().cpu().numpy()
+    k = -(-a.nbytes // budget)
+    if k > 1:
+        a = a.reshape(-1)[::k]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, name + ".npy"), a)
+    log(f"wrote {os.path.join(path, name + '.npy')}: {a.shape} float32" + (f" (1 in {k} elements)" if k > 1 else ""))
 
 
 T_START = time.perf_counter()
@@ -250,8 +267,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--replicas", action="store_true", help="N > 1: independent clips per GPU instead of one frame-sharded clip")
     ap.add_argument("--no-clip", action="store_true", help="skip the whole-clip pipeline (configs[4]) measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the eps of the last timed step as DIR/eps.npy (float32)")
     ap.add_argument("--cpu-baseline-worker", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -275,7 +297,7 @@ def main():
         # the reference's algorithm on the host cores (oracle port; the product package is never imported on this arm)
         if rank != 0:
             return
-        steps, warmup = max(1, min(args.steps, 20)), max(1, min(args.warmup, 5))
+        steps, warmup = args.steps, max(1, min(args.warmup, 5))
         cb, sec = cpu_baseline_run(sd_cpu, steps, warmup)
         cb["cfg1"] = cpu_cfg1_run(sd_cpu)
         line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": "steps/s", "n_gpus": args.gpus,
@@ -342,6 +364,8 @@ def main():
         ms_total = float(tt.item())
     ms_per_step = ms_total / args.steps
     value = args.gpus * 1000.0 / ms_per_step
+    if args.dump_outputs:                         # out_d holds the eps of the last timed step
+        dump_output(args.dump_outputs, "eps" if world == 1 else f"eps_rank{rank}", out_d, DUMP_BYTES // world)
     comm = None
     if sharded:
         # stream time spent in the sharding collectives (CUDA events around them on the compute stream: they are serialised with the

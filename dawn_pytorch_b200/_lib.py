@@ -64,6 +64,8 @@ def _load():
     lib.dawn_unet_ddim_step.argtypes = [vp, fp, fp, fp, ctypes.c_int64] + [ctypes.c_float] * 6 + [vp, vp]
     lib.dawn_unet_sampler_capture.argtypes = [vp, fp, fp, fp, vp, ctypes.POINTER(ctypes.c_float), ctypes.c_int, ctypes.c_float, vp]
     lib.dawn_unet_sampler_launch.argtypes = [vp, vp]
+    lib.dawn_unet_ddpm_step.argtypes = [vp, fp, fp, fp, ctypes.c_int64, fp, ctypes.c_float, vp, vp]
+    lib.dawn_unet_ddpm_capture.argtypes = [vp, fp, fp, fp, vp, vp, vp, ctypes.c_int, ctypes.c_float, vp]
     ip = ctypes.POINTER(ctypes.c_int)
     lib.dawn_lfg_create.argtypes = [ctypes.POINTER(DawnLfgCfg), ctypes.POINTER(vp)]
     lib.dawn_lfg_destroy.argtypes = [vp]
@@ -92,6 +94,7 @@ EXPORTS = ["dawn_unet_create", "dawn_unet_destroy", "dawn_unet_set_param", "dawn
            "dawn_unet_set_num_frames", "dawn_nccl_unique_id", "dawn_unet_init_shard", "dawn_unet_shard_ipc_export", "dawn_unet_shard_ipc_import", "dawn_unet_set_clip_invariants", "dawn_unet_forward",
            "dawn_unet_forward_x3", "dawn_unet_forward_host", "dawn_unet_set_tap", "dawn_unet_tap_shape",
            "dawn_unet_profile_enable", "dawn_unet_profile_read", "dawn_unet_last_launch_count", "dawn_unet_workspace_bytes", "dawn_ddim_step", "dawn_unet_ddim_step", "dawn_unet_sampler_capture", "dawn_unet_sampler_launch",
+           "dawn_unet_ddpm_step", "dawn_unet_ddpm_capture",
            "dawn_selftest_tc_gemm", "dawn_selftest_attention", "dawn_selftest_temporal_tc", "dawn_temporal_tc_plan", "dawn_last_error", "dawn_build_info"]
 
 

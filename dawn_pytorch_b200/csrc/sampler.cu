@@ -1,5 +1,6 @@
-// DDIM update around the denoising UNet (reference U:1169-1205): x0 prediction, dynamic thresholding with the exact
-// 0.9-quantile of |x0| over the whole clip (torch.quantile semantics, linear interpolation), and the eta-noise update.
+// DDIM and ancestral DDPM updates around the denoising UNet (reference U:1169-1205 and U:1072-1121): x0 prediction, dynamic
+// thresholding with the exact 0.9-quantile of |x0| over the whole clip (torch.quantile semantics, linear interpolation), and
+// the eta-noise (DDIM) or posterior-mean + sigma-noise (DDPM) update.  Both steps share the same select chain.
 // Everything stays on the device: no host synchronisation inside a sampling step.
 #include "common.cuh"
 #include "sampler.cuh"
@@ -14,9 +15,12 @@
 namespace dawn {
 namespace {
 
-// keys[i] = |ca * x - cb * eps|  (x0 magnitude; non-negative floats order like their bit patterns)
-__global__ void x0_abs_kernel(const float* __restrict__ x, const float* __restrict__ eps, float ca, float cb, long long n,
-                              uint32_t* __restrict__ keys) {
+// keys[i] = |ca * x - cb * eps|  (x0 magnitude; non-negative floats order like their bit patterns).  kDevCoef: ca, cb are
+// read from cab[0..1] in device memory (the DDPM step, whose per-step scalars a replayed graph cannot bake).
+template <bool kDevCoef>
+__global__ void x0_abs_kernel(const float* __restrict__ x, const float* __restrict__ eps, float ca, float cb,
+                              const float* __restrict__ cab, long long n, uint32_t* __restrict__ keys) {
+  if (kDevCoef) { ca = cab[0]; cb = cab[1]; }
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
     keys[i] = __float_as_uint(fabsf(ca * x[i] - cb * eps[i]));
 }
@@ -109,48 +113,103 @@ __global__ void ddim_update_kernel(float* __restrict__ x, const float* __restric
   }
 }
 
+// x = c1 * clamp(x0, -s, s)/s + c2 * x + sigma * noise with x0 = ca*x - cb*eps  (U:1072-1085, 1113-1121); coef = {ca, cb, c1,
+// c2, sigma} in device memory.  sigma is 0 at t = 0 (the reference's nonzero_mask), where the noise is not read at all.
+__global__ void ddpm_update_kernel(float* __restrict__ x, const float* __restrict__ eps, const float* __restrict__ noise,
+                                   const float* __restrict__ s_ptr, const float* __restrict__ coef, long long n, int clamp) {
+  const float s = s_ptr ? *s_ptr : 1.0f;
+  const float ca = coef[0], cb = coef[1], c1 = coef[2], c2 = coef[3], sigma = coef[4];
+  const bool add_noise = noise != nullptr && sigma != 0.0f;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const float xi = x[i];
+    float x0 = ca * xi - cb * eps[i];
+    if (clamp) x0 = fminf(fmaxf(x0, -s), s) / s;
+    float v = c1 * x0 + c2 * xi;
+    if (add_noise) v += sigma * noise[i];
+    x[i] = v;
+  }
+}
+
+// slot <- table row *cursor, ++*cursor: one step of a replayed DDPM segment picks up its time index and coefficients
+__global__ void ddpm_advance_kernel(const uint32_t* __restrict__ table, int* __restrict__ cursor, uint32_t* __restrict__ slot) {
+  const int r = *cursor;
+  for (int i = 0; i < kDdpmRowWords; ++i) slot[i] = table[(size_t)r * kDdpmRowWords + i];
+  *cursor = r + 1;
+}
+
+int grid_blocks(long long n, int threads) { return (int)std::min<long long>((n + threads - 1) / threads, 148LL * 8); }
+
+// The threshold s of one step: the q-quantile of |x0| over the n_global values of the WHOLE clip.  With a frame-sharded clip
+// every rank histograms its own keys and the 256-bin digit histograms (4 passes), the count <= v and the min key above v are
+// all-reduced through `red`, so every rank walks the identical radix-select and ends with the bit-identical threshold
+// (SURVEY 8e-iii).  ca, cb by value, or (cab != nullptr) from device memory.  Writes *s_ptr = the device address of s, or
+// nullptr when q <= 0 (no dynamic threshold).
+int select_threshold(const float* x, const float* eps, float ca, float cb, const float* cab, int64_t n_local, int64_t n_global,
+                     float q, void* scratch, cudaStream_t st, const DdimReduce* red, const float** s_ptr) {
+  *s_ptr = nullptr;
+  if (!(q > 0.f)) return 0;
+  const long long n = n_local;
+  const int threads = 256;
+  const int blocks = grid_blocks(n, threads);
+  // scratch layout (32-bit words): [0,4) select state | [4,260) histogram | [260,262) count_le (u64) | 262 min_gt | 263 s | [512, 512+n) keys
+  uint32_t* base = (uint32_t*)scratch;
+  uint32_t* state = base;
+  unsigned int* hist = base + 4;
+  unsigned long long* count_le = (unsigned long long*)(base + 260);
+  unsigned int* min_gt = base + 262;
+  float* s_out = (float*)(base + 263);
+  uint32_t* keys = base + 512;
+  // torch.quantile: ranks = q * (n - 1) evaluated in fp32 (ATen quantile_compute), lerp between floor and ceil
+  const float rank_f = q * (float)(n_global - 1);
+  const long long lo = (long long)floorf(rank_f), hi = (long long)ceilf(rank_f);
+  const float w = rank_f - floorf(rank_f);
+  select_init_kernel<<<1, 256, 0, st>>>(state, hist, count_le, min_gt, (unsigned long long)lo);
+  if (cab) x0_abs_kernel<true><<<blocks, threads, 0, st>>>(x, eps, 0.f, 0.f, cab, n, keys);
+  else x0_abs_kernel<false><<<blocks, threads, 0, st>>>(x, eps, ca, cb, nullptr, n, keys);
+  for (int shift = 24; shift >= 0; shift -= 8) {
+    radix_hist_kernel<<<blocks, 256, 0, st>>>(keys, n, state, shift, hist);
+    if (red) DAWN_TRY(red->sum_u32(red->ctx, hist, 256, st));
+    radix_pick_kernel<<<1, 32, 0, st>>>(state, shift, hist);
+  }
+  next_stat_kernel<<<blocks, threads, 0, st>>>(keys, n, state, count_le, min_gt);
+  if (red) {
+    DAWN_TRY(red->sum_u64(red->ctx, count_le, 1, st));
+    DAWN_TRY(red->min_u32(red->ctx, min_gt, 1, st));
+  }
+  threshold_kernel<<<1, 1, 0, st>>>(state, count_le, min_gt, lo, hi, w, s_out);
+  *s_ptr = s_out;
+  return 0;
+}
+
 }  // namespace
 
-// One DDIM update in place on x (n_local floats of this rank's frames of the (3, F, h, w) latent).  The dynamic threshold
-// is the q-quantile of |x0| over the n_global values of the WHOLE clip: with a frame-sharded clip every rank histograms
-// its own keys and the 256-bin digit histograms (4 passes), the count <= v and the min key above v are all-reduced through
-// `red`, so every rank walks the identical radix-select and ends with the bit-identical threshold (SURVEY 8e-iii).
+// One DDIM update in place on x (n_local floats of this rank's frames of the (3, F, h, w) latent); the threshold is
+// select_threshold's clip-wide quantile.
 int ddim_step_impl(float* x, const float* eps, const float* noise, int64_t n_local, int64_t n_global, float ca, float cb,
                    float sqrt_an, float c, float sigma, float q, void* scratch, cudaStream_t st, const DdimReduce* red) {
   if (!x || !eps || !scratch || n_local <= 0 || n_global < n_local) { set_last_error("dawn_ddim_step: bad argument"); return -1; }
-  const long long n = n_local;
-  const int threads = 256;
-  int blocks = (int)std::min<long long>((n + threads - 1) / threads, 148LL * 8);
-  float* s_ptr = nullptr;
-  if (q > 0.f) {
-    // scratch layout (32-bit words): [0,4) select state | [4,260) histogram | [260,262) count_le (u64) | 262 min_gt | 263 s | [512, 512+n) keys
-    uint32_t* base = (uint32_t*)scratch;
-    uint32_t* state = base;
-    unsigned int* hist = base + 4;
-    unsigned long long* count_le = (unsigned long long*)(base + 260);
-    unsigned int* min_gt = base + 262;
-    float* s_out = (float*)(base + 263);
-    uint32_t* keys = base + 512;
-    // torch.quantile: ranks = q * (n - 1) evaluated in fp32 (ATen quantile_compute), lerp between floor and ceil
-    const float rank_f = q * (float)(n_global - 1);
-    const long long lo = (long long)floorf(rank_f), hi = (long long)ceilf(rank_f);
-    const float w = rank_f - floorf(rank_f);
-    select_init_kernel<<<1, 256, 0, st>>>(state, hist, count_le, min_gt, (unsigned long long)lo);
-    x0_abs_kernel<<<blocks, threads, 0, st>>>(x, eps, ca, cb, n, keys);
-    for (int shift = 24; shift >= 0; shift -= 8) {
-      radix_hist_kernel<<<blocks, 256, 0, st>>>(keys, n, state, shift, hist);
-      if (red) DAWN_TRY(red->sum_u32(red->ctx, hist, 256, st));
-      radix_pick_kernel<<<1, 32, 0, st>>>(state, shift, hist);
-    }
-    next_stat_kernel<<<blocks, threads, 0, st>>>(keys, n, state, count_le, min_gt);
-    if (red) {
-      DAWN_TRY(red->sum_u64(red->ctx, count_le, 1, st));
-      DAWN_TRY(red->min_u32(red->ctx, min_gt, 1, st));
-    }
-    threshold_kernel<<<1, 1, 0, st>>>(state, count_le, min_gt, lo, hi, w, s_out);
-    s_ptr = s_out;
-  }
-  ddim_update_kernel<<<blocks, threads, 0, st>>>(x, eps, noise, s_ptr, ca, cb, sqrt_an, c, sigma, n, q < 0.f ? 0 : 1);
+  const float* s_ptr = nullptr;
+  DAWN_TRY(select_threshold(x, eps, ca, cb, nullptr, n_local, n_global, q, scratch, st, red, &s_ptr));
+  ddim_update_kernel<<<grid_blocks(n_local, 256), 256, 0, st>>>(x, eps, noise, s_ptr, ca, cb, sqrt_an, c, sigma, n_local,
+                                                                q < 0.f ? 0 : 1);
+  DAWN_LAUNCH_OK();
+  return 0;
+}
+
+// One ancestral DDPM update in place on x: the same select as the DDIM step, then the posterior update with the five
+// coefficients {ca, cb, c1, c2, sigma} read from coef (device memory).
+int ddpm_step_impl(float* x, const float* eps, const float* noise, int64_t n_local, int64_t n_global, const float* coef, float q,
+                   void* scratch, cudaStream_t st, const DdimReduce* red) {
+  if (!x || !eps || !coef || !scratch || n_local <= 0 || n_global < n_local) { set_last_error("dawn_ddpm_step: bad argument"); return -1; }
+  const float* s_ptr = nullptr;
+  DAWN_TRY(select_threshold(x, eps, 0.f, 0.f, coef, n_local, n_global, q, scratch, st, red, &s_ptr));
+  ddpm_update_kernel<<<grid_blocks(n_local, 256), 256, 0, st>>>(x, eps, noise, s_ptr, coef, n_local, q < 0.f ? 0 : 1);
+  DAWN_LAUNCH_OK();
+  return 0;
+}
+
+int launch_ddpm_advance(const void* table, int* cursor, void* slot, cudaStream_t st) {
+  ddpm_advance_kernel<<<1, 1, 0, st>>>((const uint32_t*)table, cursor, (uint32_t*)slot);
   DAWN_LAUNCH_OK();
   return 0;
 }

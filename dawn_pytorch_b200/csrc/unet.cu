@@ -1697,6 +1697,52 @@ int dawn_unet_sampler_capture(dawn_unet* h, float* x, float* eps, const float* n
   return 0;
 }
 
+// Ancestral DDPM update of this handle's frames (reference p_sample U:1113-1121): the DDIM step's select (clip-wide when
+// sharded), then the posterior update with {ca, cb, c1, c2, sigma} read from coef (device memory).
+int dawn_unet_ddpm_step(dawn_unet* h, float* x, const float* eps, const float* noise, int64_t n_local, const float* coef, float q,
+                        void* scratch, void* stream) {
+  DAWN_CHECK(h, "null handle");
+  if (h->sh_nranks <= 1 || !h->sh_comm)
+    return ddpm_step_impl(x, eps, noise, n_local, n_local, coef, q, scratch, (cudaStream_t)stream, nullptr);
+  DdimReduce red{(void*)h->sh_comm, red_sum_u32, red_sum_u64, red_min_u32};
+  return ddpm_step_impl(x, eps, noise, n_local, n_local * h->sh_nranks, coef, q, scratch, (cudaStream_t)stream, &red);
+}
+
+// One SEGMENT of the ancestral loop (ksteps x [advance + forward_x3 + DDPM update]) as the handle's sampler graph.  The graph
+// bakes no per-step value: each step first copies table row *cursor into slot and increments *cursor, the forward reads t
+// from slot and the update its coefficients, so replaying the segment T / ksteps times walks the whole table.  Step j of a
+// segment reads noise slice j of noise_ring (ksteps x n floats), which the caller refills before every launch.
+int dawn_unet_ddpm_capture(dawn_unet* h, float* x, float* eps, const float* noise_ring, const void* table, int* cursor, void* slot,
+                           int ksteps, float q, void* scratch) {
+  DAWN_CHECK(h && x && eps && noise_ring && table && cursor && slot && scratch && ksteps >= 1, "bad argument");
+  DAWN_CHECK(h->F > 0 && h->have_invariants, "set_clip_invariants must precede ddpm_capture");
+  DAWN_CHECK(!h->prof_on, "disable profiling before capturing the sampler graph");
+  drop_sampler_graph(h);
+  if (!h->samp_stream) DAWN_CUDA_OK(cudaStreamCreateWithFlags(&h->samp_stream, cudaStreamNonBlocking));
+  const int64_t n = (int64_t)(h->cfg.out_grid_dim + h->cfg.out_conf_dim) * h->F * h->H * h->W;
+  const int64_t* t_slot = (const int64_t*)slot;
+  const float* coef_slot = (const float*)slot + kDdpmCoefWord;
+  cudaStream_t st = h->samp_stream;
+  DAWN_CUDA_OK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+  int rc = 0;
+  for (int k = 0; k < ksteps && rc == 0; ++k) {
+    rc = launch_ddpm_advance(table, cursor, slot, st);
+    if (rc == 0) rc = dawn_unet_forward_x3(h, x, t_slot, eps, st);
+    if (rc == 0) rc = dawn_unet_ddpm_step(h, x, eps, noise_ring + (size_t)k * n, n, coef_slot, q, scratch, st);
+  }
+  cudaGraph_t graph = nullptr;
+  const cudaError_t e = cudaStreamEndCapture(st, &graph);
+  if (rc != 0) { if (graph) cudaGraphDestroy(graph); return rc; }
+  DAWN_CUDA_OK(e);
+  size_t nodes = 0;
+  cudaGraphGetNodes(graph, nullptr, &nodes);
+  const cudaError_t ei = cudaGraphInstantiate(&h->samp_exec, graph, 0);
+  cudaGraphDestroy(graph);
+  DAWN_CUDA_OK(ei);
+  h->samp_launches = (int64_t)nodes;
+  return 0;
+}
+
 int dawn_unet_sampler_launch(dawn_unet* h, void* stream) {
   DAWN_CHECK(h && h->samp_exec, "sampler_capture must precede sampler_launch (a geometry change drops the graph)");
   DAWN_CHECK(h->have_invariants, "set_clip_invariants must precede sampler_launch");

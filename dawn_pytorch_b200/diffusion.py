@@ -1,12 +1,12 @@
 """Drop-in replacement for the reference's `GaussianDiffusion` / `DynamicNfGaussianDiffusion` sampler
 (DM_3/modules/video_flow_diffusion_multiGPU_v0_crema_plus_faceemb_ca_multi_test.py:988-1313) around the CUDA UNet:
 same constructor keywords, the same 12 schedule buffers (so `diffusion.load_state_dict(checkpoint['diffusion'])`,
-unified_video_generator.py:527-528, fills `denoise_fn.*` and the buffers), `sample(fea, bbox_mask, cond, cond_scale)`
-and `ddim_sample`.  Training entry points (`forward`, `p_losses`) are out of scope and raise.
+unified_video_generator.py:527-528, fills `denoise_fn.*` and the buffers), `sample(fea, bbox_mask, cond, cond_scale)`,
+`ddim_sample` and the ancestral `p_sample_loop`.  Training entry points (`forward`, `p_losses`) are out of scope and raise.
 
 The sampling loop keeps the clip on the device: the 272 feature channels and the conditioning are handed to the UNet
-once per clip (`set_clip_invariants`), each step is `forward_x3` + one fused `dawn_ddim_step` (x0, exact clip-wide
-0.9-quantile dynamic threshold, eta-noise update) with no host synchronisation.
+once per clip (`set_clip_invariants`), each step is `forward_x3` + one fused `dawn_ddim_step` / `dawn_unet_ddpm_step` (x0,
+exact clip-wide 0.9-quantile dynamic threshold, eta-noise or posterior update) with no host synchronisation.
 """
 import ctypes
 
@@ -15,6 +15,10 @@ import torch.nn.functional as F
 from torch import nn
 
 from ._lib import check, lib
+
+# Steps per captured DDPM segment: the ancestral loop (T = 1000 as DAWN configures it) replays one K-step graph T // K times
+# and runs the last T mod K steps eagerly.  K = 20 gives the graph the node count of the 20-step DDIM graph.
+DDPM_SEGMENT_STEPS = 20
 
 
 def _cosine_beta_schedule(timesteps, s=0.008):
@@ -85,14 +89,40 @@ class GaussianDiffusion(nn.Module):
         c = ((1 - alpha_next) - sigma ** 2).sqrt()
         return ca, cb, float(alpha_next.sqrt()), float(c), float(sigma)
 
+    def ddpm_coefficients(self, t):
+        """Host-side scalars of one ancestral step, {ca, cb, c1, c2, sigma}, with the reference's fp32 torch arithmetic:
+        x0 = ca*x - cb*eps (U:1072-1076), mean = c1*x0 + c2*x (U:1078-1085), and sigma = nonzero_mask *
+        exp(0.5 * posterior_log_variance_clipped[t]) (U:1118-1121), which is 0 at t = 0.  The five schedule buffers are
+        copied to the host once."""
+        tabs = getattr(self, "_host_post", None)
+        stamp = (self.posterior_log_variance_clipped.data_ptr(), self.posterior_log_variance_clipped._version)
+        if tabs is None or tabs[-1] != stamp:
+            tabs = tuple(b.detach().cpu() for b in (self.sqrt_recip_alphas_cumprod, self.sqrt_recipm1_alphas_cumprod,
+                                                    self.posterior_mean_coef1, self.posterior_mean_coef2,
+                                                    self.posterior_log_variance_clipped)) + (stamp,)
+            self._host_post = tabs
+        sra, srm1, c1, c2, lv = tabs[:5]
+        nonzero_mask = 1 - (torch.tensor([t]) == 0).float()
+        sigma = nonzero_mask * (0.5 * lv[t:t + 1]).exp()
+        return float(sra[t]), float(srm1[t]), float(c1[t]), float(c2[t]), float(sigma)
+
+    def ddpm_table(self, times):
+        """Per-loop table of the ancestral loop, one row of eight 32-bit words per step: {t (int64), ca, cb, c1, c2, sigma,
+        unused} (the row layout `dawn_unet_ddpm_capture` reads).  int64 (len(times), 4) on the host."""
+        rows = torch.zeros((len(times), 4), dtype=torch.int64)
+        words = rows.view(torch.float32)
+        for k, t in enumerate(times):
+            rows[k, 0] = int(t)
+            words[k, 2:7] = torch.tensor(self.ddpm_coefficients(int(t)), dtype=torch.float32)
+        return rows
+
     @torch.no_grad()
     def sample(self, fea, bbox_mask, cond=None, cond_scale=1., batch_size=16):
         batch_size = cond.shape[0] if cond is not None else batch_size
-        if not self.is_ddim_sampling:
-            raise NotImplementedError("only DDIM sampling (sampling_timesteps < timesteps) is implemented, as DAWN configures it")
+        sample_fn = self.ddim_sample if self.is_ddim_sampling else self.p_sample_loop          # U:1150
         fea = torch.cat([fea, bbox_mask], dim=1)
-        return self.ddim_sample(fea, (batch_size, self.channels, self.num_frames, fea.shape[-1], fea.shape[-1]), cond=cond,
-                                cond_scale=cond_scale)
+        return sample_fn(fea, (batch_size, self.channels, self.num_frames, fea.shape[-1], fea.shape[-1]), cond=cond,
+                         cond_scale=cond_scale)
 
     @torch.no_grad()
     def ddim_sample(self, fea, shape, cond=None, cond_scale=1., clip_denoised=True, noise_fn=None, pairs=None,
@@ -115,12 +145,7 @@ class GaussianDiffusion(nn.Module):
         n = ch * Fr * h * w
         # q > 0: dynamic threshold; q = 0: static clamp to [-1, 1]; q < 0: no clamp at all (clip_denoised=False, U:1183)
         q = (float(self.dynamic_thres_percentile) if self.use_dynamic_thres else 0.0) if clip_denoised else -1.0
-        if tuple(shape[1:]) != (self.channels,) + tuple(shape[2:]) or fea.shape[0] != b or (cond is not None and cond.shape[0] != b):
-            raise ValueError(f"ddim_sample: shape {tuple(shape)} does not match fea {tuple(fea.shape)} / cond "
-                             f"{None if cond is None else tuple(cond.shape)} (batch) or channels {self.channels}")
-        if tuple(fea.shape[-2:]) != (h, w) or (cond is not None and cond.shape[1] != Fr):
-            raise ValueError(f"ddim_sample: fea {tuple(fea.shape)} / cond {None if cond is None else tuple(cond.shape)} do not "
-                             f"match the sample shape {tuple(shape)}")
+        self._check_sample_args("ddim_sample", fea, shape, cond)
         st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
         guided = cond_scale != 1 and getattr(unet, "has_cond", True)
         if use_graph:
@@ -155,6 +180,118 @@ class GaussianDiffusion(nn.Module):
                                               ctypes.c_void_p(noise.data_ptr()) if noise is not None else None, n,
                                               ca, cb, san, c, sigma, q,
                                               ctypes.c_void_p(scratch.data_ptr()), st), "dawn_unet_ddim_step")
+        return img
+
+    def _check_sample_args(self, what, fea, shape, cond):
+        b, ch, Fr, h, w = shape
+        if tuple(shape[1:]) != (self.channels,) + tuple(shape[2:]) or fea.shape[0] != b or (cond is not None and cond.shape[0] != b):
+            raise ValueError(f"{what}: shape {tuple(shape)} does not match fea {tuple(fea.shape)} / cond "
+                             f"{None if cond is None else tuple(cond.shape)} (batch) or channels {self.channels}")
+        if tuple(fea.shape[-2:]) != (h, w) or (cond is not None and cond.shape[1] != Fr):
+            raise ValueError(f"{what}: fea {tuple(fea.shape)} / cond {None if cond is None else tuple(cond.shape)} do not "
+                             f"match the sample shape {tuple(shape)}")
+
+    @torch.no_grad()
+    def p_sample_loop(self, fea, shape, cond=None, cond_scale=1., noise_fn=None, use_graph=False, seed=None, times=None):
+        """Ancestral DDPM sampling (reference p_sample_loop / p_sample, U:1113-1135): one UNet forward and one posterior update
+        per t = T-1 ... 0, always clip_denoised (static clamp, or the dynamic threshold when use_dynamic_thres).
+
+        fea, shape, cond, cond_scale, noise_fn, seed as in `ddim_sample`: noise_fn(step_index, shape) supplies the start image
+        (step -1) and the noise of loop step k; it is called only for steps with t > 0, so the eager and graph paths draw the
+        same sequence.  times: the t of every loop step (default reversed(range(num_timesteps))).
+        use_graph: capture DDPM_SEGMENT_STEPS steps once as a CUDA graph (`dawn_unet_ddpm_capture`) and replay it
+        T // DDPM_SEGMENT_STEPS times per clip, the graph reading t and the coefficients from a device table; the last
+        T mod DDPM_SEGMENT_STEPS steps run eagerly.  Classifier-free guidance (cond_scale != 1) runs eagerly.
+        Frame-sharded UNet: as `ddim_sample` (clip-wide quantile, the rank's slice of one clip-wide noise stream)."""
+        device = self.betas.device
+        b, ch, Fr, h, w = shape
+        unet = self.denoise_fn
+        times = list(reversed(range(self.num_timesteps))) if times is None else [int(t) for t in times]
+        self._check_sample_args("p_sample_loop", fea, shape, cond)
+        draw = noise_fn if noise_fn is not None else self._default_noise(unet, device, seed)
+        img = draw(-1, shape).to(device).contiguous()
+        n = ch * Fr * h * w
+        # p_sample always clips (U:1113): q > 0 dynamic threshold, q = 0 static clamp to [-1, 1]
+        q = float(self.dynamic_thres_percentile) if self.use_dynamic_thres else 0.0
+        table = self.ddpm_table(times)
+        st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+        guided = cond_scale != 1 and getattr(unet, "has_cond", True)
+        if use_graph:
+            if guided:
+                raise NotImplementedError("use_graph captures the cond_scale = 1 loop (DAWN's shipped setting); "
+                                          "classifier-free guidance runs eagerly")
+            return self._ddpm_sample_graph(unet, fea, cond, img, times, table, draw, q, st)
+        tab = table.to(device)
+        scratch = torch.empty(n + 512, dtype=torch.int32, device=device)
+        eps = torch.empty((ch, Fr, h, w), device=device)
+        eps_null = torch.empty_like(eps) if guided else None
+        for i in range(b):
+            unet.update_num_frames(Fr)
+            if not guided:
+                unet.set_clip_invariants(fea[i], cond[i])
+            x = img[i]
+            for k, t in enumerate(times):
+                t_dev = tab[k, 0:1]
+                if guided:
+                    # two hoisted forwards per step, cond then the all-zero null cond, exactly as guided ddim_sample
+                    unet.set_clip_invariants(fea[i], cond[i])
+                    unet.forward_x3(x, t_dev, eps)
+                    unet.set_clip_invariants(fea[i], torch.zeros_like(cond[i]))
+                    unet.forward_x3(x, t_dev, eps_null)
+                    torch.add(eps_null, eps - eps_null, alpha=float(cond_scale), out=eps)
+                else:
+                    unet.forward_x3(x, t_dev, eps)
+                self._ddpm_update(unet, x, eps, tab, k, t, draw, q, scratch, st)
+        return img
+
+    @staticmethod
+    def _ddpm_update(unet, x, eps, tab, k, t, draw, q, scratch, st):
+        """dawn_unet_ddpm_step for loop step k, coefficients read from row k of the device table; no draw at t = 0."""
+        noise = draw(k, tuple(x.shape)).to(x.device).contiguous() if t > 0 else None
+        coef = ctypes.c_void_p(tab.data_ptr() + k * tab.stride(0) * tab.element_size() + 8)     # row k, word 2
+        check(lib.dawn_unet_ddpm_step(unet._handle, ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(eps.data_ptr()),
+                                      ctypes.c_void_p(noise.data_ptr()) if noise is not None else None, x.numel(), coef, q,
+                                      ctypes.c_void_p(scratch.data_ptr()), st), "dawn_unet_ddpm_step")
+
+    def _ddpm_sample_graph(self, unet, fea, cond, img, times, table, draw, q, st):
+        b, ch, Fr, h, w = img.shape
+        device, n, T, K = img.device, ch * Fr * h * w, len(times), DDPM_SEGMENT_STEPS
+        nseg = T // K
+        key = ("ddpm", Fr, h, w, T, K, q, device.index)
+        g = getattr(self, "_graph", None)
+        unet.update_num_frames(Fr)
+        if g is None or g["key"] != key or (nseg and g["gen"] != unet.graph_generation()):
+            g = dict(key=key, x=torch.empty((ch, Fr, h, w), device=device), eps=torch.empty((ch, Fr, h, w), device=device),
+                     ring=torch.empty((K, ch, Fr, h, w), device=device) if nseg else None,
+                     table=torch.empty((T, 4), dtype=torch.int64, device=device),
+                     cursor=torch.zeros(1, dtype=torch.int32, device=device), slot=torch.zeros(4, dtype=torch.int64, device=device),
+                     scratch=torch.empty(n + 512, dtype=torch.int32, device=device), gen=None)
+            if nseg:
+                unet.set_clip_invariants(fea[0], cond[0])
+                torch.cuda.synchronize(device)
+                unet.claim_graph_slot()
+                check(lib.dawn_unet_ddpm_capture(unet._handle, ctypes.c_void_p(g["x"].data_ptr()), ctypes.c_void_p(g["eps"].data_ptr()),
+                                                 ctypes.c_void_p(g["ring"].data_ptr()), ctypes.c_void_p(g["table"].data_ptr()),
+                                                 ctypes.c_void_p(g["cursor"].data_ptr()), ctypes.c_void_p(g["slot"].data_ptr()),
+                                                 K, q, ctypes.c_void_p(g["scratch"].data_ptr())), "dawn_unet_ddpm_capture")
+                g["gen"] = unet.graph_generation()
+            self._graph = g
+        g["table"].copy_(table)
+        shp = (ch, Fr, h, w)
+        for i in range(b):
+            unet.set_clip_invariants(fea[i], cond[i])
+            g["x"].copy_(img[i])
+            g["cursor"].zero_()
+            for m in range(nseg):
+                for j in range(K):              # the ring holds exactly this segment's draws; stream-ordered after the last launch
+                    k = m * K + j
+                    if times[k] > 0:
+                        g["ring"][j].copy_(draw(k, shp))
+                check(lib.dawn_unet_sampler_launch(unet._handle, st), "dawn_unet_sampler_launch")
+            for k in range(nseg * K, T):        # remainder: the same tables, eagerly
+                unet.forward_x3(g["x"], g["table"][k, 0:1], g["eps"])
+                self._ddpm_update(unet, g["x"], g["eps"], g["table"], k, times[k], draw, q, g["scratch"], st)
+            img[i].copy_(g["x"])
         return img
 
     @staticmethod
@@ -196,6 +333,7 @@ class GaussianDiffusion(nn.Module):
                 assert (t_next > 0) == (k < ns - 1), "only the last DDIM step ends at t = 0 (reference :1201)"
             unet.set_clip_invariants(fea[0], cond[0])
             torch.cuda.synchronize(device)
+            unet.claim_graph_slot()
             check(lib.dawn_unet_sampler_capture(unet._handle, ctypes.c_void_p(g["x"].data_ptr()), ctypes.c_void_p(g["eps"].data_ptr()),
                                                 ctypes.c_void_p(g["noise"].data_ptr()), ctypes.c_void_p(g["t_all"].data_ptr()),
                                                 coef, ns, q, ctypes.c_void_p(g["scratch"].data_ptr())), "dawn_unet_sampler_capture")

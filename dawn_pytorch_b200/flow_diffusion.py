@@ -4,7 +4,7 @@ the object `unified_video_generator.py:513-531` builds and calls `update_num_fra
 
 Same attribute names (`generator`, `unet`, `diffusion`, `face_loc_emb`), so `model.diffusion.load_state_dict(checkpoint['diffusion'])`
 (UVG:527-528) and `generator.load_state_dict(checkpoint['generator'])` (FD:120) work unchanged; `sample_one_video` keeps its
-signature and output dictionary.  Underneath: the source encoder, the 20-step DDIM loop and the frame decoder are the CUDA paths of
+signature and output dictionary.  Underneath: the source encoder, the DDIM (or ancestral DDPM) loop and the frame decoder are the CUDA paths of
 this package (LfgGenerator, DynamicNfGaussianDiffusion over DynamicNfUnet3D) — one batched decode instead of a Python loop over
 frames (FD:375-383).  Training-only members (region / background predictors, VGG loss, `forward`) are out of scope and absent.
 """
@@ -136,10 +136,10 @@ class FlowDiffusion(nn.Module):
         b = fea.shape[0]
         fea272 = torch.cat([fea, bbox_mask], dim=1)                                     # GaussianDiffusion.sample, U:1151
         h, w = fea272.shape[-2:]
-        if not self.diffusion.is_ddim_sampling:           # the reference's sample() would run p_sample_loop here (U:1137-1154)
-            raise NotImplementedError("only DDIM sampling (sampling_timesteps < timesteps) is implemented, as DAWN configures it")
-        pred = self.diffusion.ddim_sample(fea272, (b, self.diffusion.channels, self.diffusion.num_frames, h, w), cond=ref_text,
-                                          cond_scale=cond_scale, noise_fn=noise_fn, use_graph=use_graph)
+        # DDIM when sampling_timesteps < timesteps, else the ancestral loop, as the reference's sample() picks (U:1150)
+        sample_fn = self.diffusion.ddim_sample if self.diffusion.is_ddim_sampling else self.diffusion.p_sample_loop
+        pred = sample_fn(fea272, (b, self.diffusion.channels, self.diffusion.num_frames, h, w), cond=ref_text,
+                         cond_scale=cond_scale, noise_fn=noise_fn, use_graph=use_graph)
         if self.use_residual_flow:
             raise NotImplementedError("use_residual_flow=True is not used by the shipped configs (FD:362-364)")
         out["sample_vid_grid"] = pred[:, :2]                                            # FD:366

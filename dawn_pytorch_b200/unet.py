@@ -403,6 +403,11 @@ class Unet3D(nn.Module):
         """Changes whenever the native handle dropped a captured sampler graph (new geometry, parameters or sharding)."""
         return (id(self._handle), getattr(self, "_gen", 0))
 
+    def claim_graph_slot(self):
+        """Call before capturing a sampler graph: the handle holds ONE (DDIM loop or DDPM segment), so a new capture invalidates
+        whatever graph another sampler cached against the previous generation."""
+        self._gen = getattr(self, "_gen", 0) + 1
+
     def forward_x3(self, x_t, time, out=None):
         """x_t (3, F, h, w) of the clip whose invariants were set; time int64 tensor (1,) on the device."""
         if self._geom is None or getattr(self, "_fea", None) is None:

@@ -106,7 +106,8 @@ int dawn_unet_tap_shape(dawn_unet* h, const char* name, int* C, int* hl, int* wl
 int dawn_unet_profile_enable(dawn_unet* h, int on);
 int dawn_unet_profile_read(dawn_unet* h, double* ms, double* flops, double* bytes, int64_t* count);
 
-/* number of kernels launched by the last forward on this handle (bench.py's gpu_launches) */
+/* number of kernels launched by the last forward on this handle (bench.py's gpu_launches); after a sampler launch, the
+ * forward launches of the DDIM graph or the node count of the DDPM segment graph */
 int64_t dawn_unet_last_launch_count(dawn_unet* h);
 /* bytes of device workspace currently held */
 int64_t dawn_unet_workspace_bytes(dawn_unet* h);
@@ -136,6 +137,27 @@ int dawn_unet_ddim_step(dawn_unet* h, float* x, const float* eps, const float* n
 int dawn_unet_sampler_capture(dawn_unet* h, float* x, float* eps, const float* noise_all, const int64_t* t_all,
                               const float* coef, int nsteps, float q, void* scratch);
 int dawn_unet_sampler_launch(dawn_unet* h, void* stream);
+
+/* One ancestral DDPM update (reference p_sample :1113-1121 over p_mean_variance / q_posterior :1072-1107), in place on x:
+ *   x0 = ca*x - cb*eps;  s as in dawn_ddim_step (q > 0: max(1, quantile_q(|x0|)), q = 0: 1, q < 0: no clamp);
+ *   x = c1 * clamp(x0,-s,s)/s + c2*x + sigma*noise
+ * coef: DEVICE pointer to {ca, cb, c1, c2, sigma} (sqrt_recip_alphas_cumprod[t], sqrt_recipm1_alphas_cumprod[t],
+ * posterior_mean_coef1[t], posterior_mean_coef2[t], (t > 0) * exp(0.5 * posterior_log_variance_clipped[t])), so a loop
+ * keeps its whole table on the device.  sigma == 0 (t = 0) reads no noise; noise may then be NULL.  Unsharded handle: the
+ * plain step; after dawn_unet_init_shard the quantile spans the whole clip exactly as in dawn_unet_ddim_step.
+ * scratch as dawn_ddim_step.  No host synchronisation. */
+int dawn_unet_ddpm_step(dawn_unet* h, float* x, const float* eps, const float* noise, int64_t n_local, const float* coef, float q,
+                        void* scratch, void* stream);
+
+/* A segment of the ancestral loop captured as the handle's sampler graph (replaces any captured DDIM loop; replay it with
+ * dawn_unet_sampler_launch).  The graph holds ksteps x [advance, forward_x3, dawn_unet_ddpm_step] and bakes no per-step value:
+ * table (device) holds one row of 8 32-bit words per loop step, {t (int64), ca, cb, c1, c2, sigma, unused}; each step copies
+ * row *cursor (device int) into slot (device, 8 words), increments *cursor, and runs the forward at slot's t and the update
+ * with slot's coefficients.  Step j of a segment adds noise_ring slice j (ksteps x 3*F*h*w floats).  Per clip: set
+ * *cursor = 0, then per segment refill noise_ring and launch; launch m runs table rows [m*ksteps, (m+1)*ksteps).  x, eps,
+ * scratch as dawn_unet_sampler_capture.  set_num_frames / commit_params / init_shard drop the graph. */
+int dawn_unet_ddpm_capture(dawn_unet* h, float* x, float* eps, const float* noise_ring, const void* table, int* cursor, void* slot,
+                           int ksteps, float q, void* scratch);
 
 /* self-test of the tcgen05 contraction kernel against the mma.sync kernel on a random k x k convolution
  * (F frames of H x W, Cin -> N channels); reports max |difference| (outputs and, if requested, GroupNorm sums). */
